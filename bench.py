@@ -294,6 +294,27 @@ def run_reference(args, wl, rank, world):
     }))
 
 
+def device_to_host(ptr, shape, typestr):
+    """Host copy of a contiguous array in the library's device memory, read through the CUDA array interface."""
+    import torch
+
+    class DeviceView:
+        __cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 3}
+    return torch.as_tensor(DeviceView(), device="cuda").cpu().numpy()
+
+
+def dump_step_outputs(out_dir, L, h, B, Cn, prefix):
+    """What the last timed step left in the model's result buffers, i.e. what sr_classify_ids hands its caller:
+    logits / probs [B, C], cls / conf [B]; float32, cls as float64 (exact for class ids)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"logits": device_to_host(L.sr_dev_logits(h), (B, Cn), "<f4"),
+              "probs": device_to_host(L.sr_dev_probs(h), (B, Cn), "<f4"),
+              "cls": device_to_host(L.sr_dev_cls(h), (B,), "<i4").astype(np.float64),
+              "conf": device_to_host(L.sr_dev_conf(h), (B,), "<f4")}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def peaks():
     try:
         return json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -510,8 +531,14 @@ def main():
     ap.add_argument("--no-text-e2e", action="store_true")
     ap.add_argument("--qps", type=float, default=100000.0, help="stream workloads: offered load of the whole job (BASELINE cfg 5: 100 k)")
     ap.add_argument("--duration", type=float, default=3.0, help="stream workloads: seconds of arrivals per phase")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (logits, probs, cls, conf) as DIR/<name>.npy; the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared array for array "
+                         "(under torchrun each rank writes DIR/rank<r>_<name>.npy)")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
+    if args.dump_outputs and (args.impl != "b200" or wl.get("kind")):
+        ap.error("--dump-outputs covers the encoder workloads of the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -599,6 +626,8 @@ def main():
     ms = ev0.elapsed_time(ev1)
     launches = L.sr_launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs:   # before anything else runs on the model: its result buffers still hold the last timed step
+        dump_step_outputs(args.dump_outputs, L, h, B, Cn, "" if world == 1 else f"rank{rank}_")
     t = torch.tensor([ms], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -51,6 +54,42 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = _run(["--impl", "reference", "--workload", "modernbert-6l-b64-s128", "--gpus", "2", "--steps", "1", "--warmup", "0"],
              env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(srlib, cuda, tmp_path):
+    """--dump-outputs: two runs with the same arguments write identical arrays, `steps` in the line is the --steps
+    asked for, and the arrays are what the host-buffer call returns to its caller for the same seeded batch."""
+    sys.path.insert(0, ROOT)
+    import bench
+    workload = "modernbert-6l-b64-s128"
+    names = ("logits", "probs", "cls", "conf")
+    runs = []
+    for i, steps in enumerate((2, 3)):
+        d = tmp_path / f"run{i}"
+        r = _run(["--workload", workload, "--steps", str(steps), "--warmup", "1", "--no-cpu-baseline", "--no-text-e2e",
+                  "--dump-outputs", str(d)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        assert sorted(os.listdir(d)) == sorted(n + ".npy" for n in names)
+        runs.append({n: np.load(d / (n + ".npy")) for n in names})
+    for n in names:
+        assert runs[0][n].dtype in (np.float32, np.float64) and np.array_equal(runs[0][n], runs[1][n]), n
+    wl = bench.WORKLOADS[workload]
+    _, wdir = bench.make_model_dir(wl, workload)
+    ids, cu = bench.make_batch(wl, 1000)
+    m = srlib.Model(wdir, device=0)
+    want = m.classify_packed(ids, cu)
+    m.close()
+    assert runs[0]["logits"].shape == (wl["batch"], wl["classes"])
+    for n in names:
+        assert np.array_equal(runs[0][n], want[n].astype(runs[0][n].dtype)), n
+
+
+def test_dump_outputs_refused_where_it_has_no_meaning(tmp_path):
+    r = _run(["--impl", "reference", "--workload", "modernbert-6l-b64-s128", "--steps", "1", "--warmup", "0",
+              "--dump-outputs", str(tmp_path / "d")])
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "d").exists()
 
 
 def test_own_arm_refuses_without_a_gpu():
