@@ -51,6 +51,12 @@ SR_API int sr_test_attention_win(const void* qkv_f16, void* out_f16, const int32
 SR_API int sr_test_attention_trace(void* dev_buf_3x4096_i64);
 SR_API int sr_test_layernorm(const float* x, int t, int h, const float* w, const float* b, float eps, float* y32,
                       void* y16);
+/* The pipeline sr_cache_topk takes for b queries over n stored rows of dim d and top-k (host only, no GPU needed):
+ * route -1 refused, 0 nothing to do (b or k <= 0), 1 empty store, 2 GEMV scores + two-stage selection (b <= 4),
+ * 3 GEMM with the fused top-8 epilogue (b > 4, k <= 8), 4 GEMM scores + two-stage selection; chunks / chunk_rows: the
+ * score chunks of routes 2 and 4; stage2_smem: shared memory of the final selection (route 3: its upper bound). */
+SR_API int sr_test_cache_topk_plan(int b, int n, int d, int k, int32_t* route, int32_t* chunks, int32_t* chunk_rows,
+                                   int64_t* stage2_smem);
 
 #ifdef __cplusplus
 }

@@ -595,6 +595,16 @@ int sr_test_attention_trace(void* dev_buf_3x4096_i64) {
 int sr_test_layernorm(const float* x, int t, int hdim, const float* w, const float* b, float eps, float* y32, void* y16) {
   return layernorm_rows(nullptr, x, t, hdim, w, b, eps, y32, static_cast<__half*>(y16));
 }
+int sr_test_cache_topk_plan(int b, int n, int d, int k, int32_t* route, int32_t* chunks, int32_t* chunk_rows,
+                            int64_t* stage2_smem) {
+  if (!route || !chunks || !chunk_rows || !stage2_smem) return -1;
+  const CacheTopkPlan p = cache_topk_plan(b, n, d, k);
+  *route = p.route;
+  *chunks = p.chunks;
+  *chunk_rows = p.chunk_rows;
+  *stage2_smem = static_cast<int64_t>(p.stage2_smem);
+  return 0;
+}
 
 #endif  // SRB_TEST_HOOKS
 

@@ -315,7 +315,29 @@ inline int chunk_rows(int B, int N) {
 
 constexpr int kFusedK = 8;        // list length of the GEMM's top-k epilogue (gemm.h EPI_TOPK)
 constexpr int kFusedLists = 320;  // upper bound of the lists per query (= 2 x CTAs launched <= 2 x SMs)
-inline bool fused_ok(int B, int k, int D) { return B > 4 && k <= kFusedK && D % 8 == 0; }
+constexpr size_t kStage2SmemMax = 200 * 1024;   // candidates select_stage2 holds in shared memory
+// A launch gets 48 KB of shared memory without the per-kernel opt-in, the static `red` array of select_stage2 /
+// merge_packed_kernel included: at exactly 48 KB of candidates the launch fails without the opt-in
+// (tests/test_cache_topk_exact_gpu.py: gemv-k64-stage2-48k, test_sharded_packed_merge_exact[96-8-64]).
+constexpr size_t kSmemDefault = 48 * 1024 - sizeof(Cand) * (kSelThreads / 32);
+
+CacheTopkPlan cache_topk_plan(int B, int N, int D, int k) {
+  CacheTopkPlan p;
+  if (B <= 0 || k <= 0) { p.route = CACHE_ROUTE_NONE; return p; }
+  if (k > 64) { p.route = CACHE_ROUTE_REFUSED; return p; }
+  if (N <= 0) { p.route = CACHE_ROUTE_EMPTY; return p; }
+  if (B > 4 && k <= kFusedK && D % 8 == 0) {
+    p.route = CACHE_ROUTE_FUSED;
+    p.stage2_smem = static_cast<size_t>(kFusedLists) * kFusedK * 8;   // bound: the GEMM reports the lists it launched
+    return p;
+  }
+  p.route = (B <= 4 && D % 8 == 0 && static_cast<size_t>(B) * D * 4 <= 48 * 1024) ? CACHE_ROUTE_GEMV : CACHE_ROUTE_GEMM;
+  p.chunk_rows = chunk_rows(B, N);
+  p.chunks = (N + p.chunk_rows - 1) / p.chunk_rows;
+  p.stage2_smem = static_cast<size_t>((N + kSegment - 1) / kSegment) * k * 8;
+  if (p.stage2_smem > kStage2SmemMax) p.route = CACHE_ROUTE_REFUSED;
+  return p;
+}
 
 size_t cache_topk_workspace_bytes(int B, int N, int k) {
   const int chunk = chunk_rows(B, N);
@@ -327,8 +349,14 @@ size_t cache_topk_workspace_bytes(int B, int N, int k) {
 
 int cache_topk(cudaStream_t stream, const __half* queries, int B, const __half* cache, const uint8_t* valid, int N,
                int D, int k, int id_offset, int* out_idx, float* out_score, void* workspace, size_t workspace_bytes) {
-  if (B <= 0 || k <= 0) return 0;
-  if (k > 64) { fprintf(stderr, "[srb200] cache_topk: k=%d unsupported (<= 64)\n", k); return -1; }
+  const CacheTopkPlan plan = cache_topk_plan(B, N, D, k);
+  if (plan.route == CACHE_ROUTE_NONE) return 0;
+  if (plan.route == CACHE_ROUTE_REFUSED) {
+    // before any launch: nothing is queued for a request that cannot be served
+    if (k > 64) fprintf(stderr, "[srb200] cache_topk: k=%d unsupported (<= 64)\n", k);
+    else fprintf(stderr, "[srb200] cache_topk: too many candidates (%zu bytes of stage-2 shared memory)\n", plan.stage2_smem);
+    return -1;
+  }
   if (workspace_bytes < cache_topk_workspace_bytes(B, N, k)) {
     fprintf(stderr, "[srb200] cache_topk: workspace too small\n");
     return -1;
@@ -340,13 +368,13 @@ int cache_topk(cudaStream_t stream, const __half* queries, int B, const __half* 
   int* cand_idx = reinterpret_cast<int*>(ws + align_up(static_cast<size_t>(B) * chunk * 4, 256));
   float* cand_score = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(cand_idx) +
                                                align_up(static_cast<size_t>(B) * segs * k * 4, 256));
-  if (N == 0) {
+  if (plan.route == CACHE_ROUTE_EMPTY) {
     select_stage2<<<B, kSelThreads, 0, stream>>>(cand_idx, cand_score, 0, k, id_offset, out_idx, out_score);
     SRB_CUDA_CHECK(cudaGetLastError());
   note_launch();
     return 0;
   }
-  if (fused_ok(B, k, D)) {
+  if (plan.route == CACHE_ROUTE_FUSED) {
     // Scores never leave the SM: the GEMM's epilogue keeps a running top-8 per (query, CTA) and only those short lists
     // are written (B x <= 148 x 8 pairs); no 1 GiB score chunks, no selection pass over them.
     int* l_idx = reinterpret_cast<int*>(ws);
@@ -368,7 +396,7 @@ int cache_topk(cudaStream_t stream, const __half* queries, int B, const __half* 
   for (int row0 = 0; row0 < N; row0 += chunk) {
     const int n = (N - row0) < chunk ? (N - row0) : chunk;
     const int n_pad = static_cast<int>(align_up(n, 64));  // cache allocation is padded to 256 rows
-    if (B <= 4 && D % 8 == 0 && static_cast<size_t>(B) * D * 4 <= 48 * 1024) {
+    if (plan.route == CACHE_ROUTE_GEMV) {
       static int num_sms = 0;
       if (!num_sms) {
         int dev = 0;
@@ -399,9 +427,8 @@ int cache_topk(cudaStream_t stream, const __half* queries, int B, const __half* 
   note_launch();
   }
   const int ncand = segs * k;
-  const size_t smem = static_cast<size_t>(ncand) * 8;
-  if (smem > 200 * 1024) { fprintf(stderr, "[srb200] cache_topk: too many candidates (%d)\n", ncand); return -1; }
-  if (smem > 48 * 1024)
+  const size_t smem = plan.stage2_smem;
+  if (smem > kSmemDefault)
     SRB_CUDA_CHECK(cudaFuncSetAttribute(select_stage2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   select_stage2<<<B, kSelThreads, smem, stream>>>(cand_idx, cand_score, ncand, k, id_offset, out_idx, out_score);
   SRB_CUDA_CHECK(cudaGetLastError());
@@ -431,6 +458,8 @@ int cache_merge_packed(cudaStream_t stream, const void* pairs, int G, int B, int
   if (B <= 0) return 0;
   const size_t smem = static_cast<size_t>(G) * k * 8;
   if (smem > 48 * 1024) { fprintf(stderr, "[srb200] cache_merge_packed: G * k = %d too large\n", G * k); return -1; }
+  if (smem > kSmemDefault)
+    SRB_CUDA_CHECK(cudaFuncSetAttribute(merge_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   merge_packed_kernel<<<B, kSelThreads, smem, stream>>>(static_cast<const int2*>(pairs), G, B, k, out_idx, out_score);
   SRB_CUDA_CHECK(cudaGetLastError());
   note_launch();

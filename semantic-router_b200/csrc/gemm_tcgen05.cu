@@ -470,9 +470,13 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
             int cidx = ocol0 + ci;
             const bool ok = cidx < p.topk_n && (!p.topk_valid || __ldg(p.topk_valid + (cidx < p.topk_n ? cidx : 0)));
             if (ok) {
+              // Insertion into the list, ordered by score and then by column.  The entries it displaces move down one
+              // place each: one that equals the next entry has the lower column and must shift past it, not fall off
+              // the end.  (With a plain `cv > tk_v[j]` a list of eight equal scores that then took a higher one lost
+              // its LOWEST column: tests/test_cache_topk_exact_gpu.py, fused-b128-same and fused-grouped-b1000-same.)
 #pragma unroll
-              for (int j = 0; j < kTopK; ++j) {   // insertion into the descending list
-                if (cv > tk_v[j]) {
+              for (int j = 0; j < kTopK; ++j) {
+                if (cv > tk_v[j] || (cv == tk_v[j] && cidx < tk_i[j])) {
                   const float tv = tk_v[j]; const int ti = tk_i[j];
                   tk_v[j] = cv; tk_i[j] = cidx;
                   cv = tv; cidx = ti;

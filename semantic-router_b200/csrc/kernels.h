@@ -96,6 +96,22 @@ int cache_topk(cudaStream_t stream, const __half* queries, int B, const __half* 
                int N, int D, int k, int id_offset, int* out_idx, float* out_score, void* workspace,
                size_t workspace_bytes);
 size_t cache_topk_workspace_bytes(int B, int N, int k);
+// Which pipeline cache_topk runs for (B, N, D, k); cache_topk branches on this and nothing else.
+enum CacheTopkRoute {
+  CACHE_ROUTE_REFUSED = -1,  // k > 64, or more stage-2 candidates than shared memory holds: error before any launch
+  CACHE_ROUTE_NONE = 0,      // B <= 0 or k <= 0: nothing to do
+  CACHE_ROUTE_EMPTY = 1,     // N == 0: every slot (-1, -inf)
+  CACHE_ROUTE_GEMV = 2,      // B <= 4: scores_small_kernel per chunk, select_stage1, select_stage2
+  CACHE_ROUTE_FUSED = 3,     // B > 4, k <= 8: EPI_TOPK GEMM lists, select_stage2
+  CACHE_ROUTE_GEMM = 4,      // otherwise: EPI_RESID GEMM scores per chunk, select_stage1, select_stage2
+};
+struct CacheTopkPlan {
+  int route = CACHE_ROUTE_NONE;
+  int chunks = 0;          // score chunks of the GEMV / GEMM routes
+  int chunk_rows = 0;      // stored rows per chunk (a multiple of the 8192-row stage-1 segment)
+  size_t stage2_smem = 0;  // dynamic shared memory of the final select_stage2 (FUSED: its upper bound)
+};
+CacheTopkPlan cache_topk_plan(int B, int N, int D, int k);
 // k-way merge of G per-shard lists [G][B,k] -> [B,k]
 int cache_merge_topk(cudaStream_t stream, const int* idx_parts, const float* score_parts, int G, int B, int k,
                      int* out_idx, float* out_score);
